@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this framework
     python bench.py --impl reference --gpus N --steps K ...  # CPU reference arm (oracle port)
+    python bench.py --gpus 1 ... --dump-outputs DIR          # also write the last timed step's outputs as DIR/<name>.npy
 
 One "step" = one energy+forces evaluation of the configured model on one synthetic frame
 (neighbour list given, built outside the timed region).  N=1 workload: BASELINE.json
@@ -93,6 +94,26 @@ def build_workload(cfg: str, dtype: str, device, scale=None):
 
 
 PARITY_TOL = {"float64": 1e-9, "float32": 1e-4, "bfloat16": 1e-3}
+DUMP_BUDGET_BYTES = 60_000_000  # --dump-outputs: all arrays together (the .npy headers come on top)
+
+
+def dump_outputs(outputs, path: str, budget: int = DUMP_BUDGET_BYTES):
+    """Write every output as <path>/<name>.npy, float64 as float64 and any other floating type as float32, so that two
+    builds can be compared array by array.  Arrays are taken smallest first, each against an even share of the bytes
+    of ``budget`` that are still left; one larger than its share keeps a sample of its rows: a fixed-seed random subset
+    in ascending row order, the same rows for every run with the same shapes."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32) for k, v in outputs.items()}
+    left = budget
+    for i, (name, t) in enumerate(sorted(arrays.items(), key=lambda kv: (kv[1].numel() * kv[1].element_size(), kv[0]))):
+        rows = t.shape[0] if t.dim() else 1
+        keep = left // (len(arrays) - i) // max(1, t.numel() // max(1, rows) * t.element_size())
+        if rows > keep:
+            t = t[torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+        left -= t.numel() * t.element_size()
+        np.save(os.path.join(path, f"{name}.npy"), t.numpy())
 
 
 def parity_check(model, out, d_cpu, kw, dtype: str, n_sample: int = 16):
@@ -190,6 +211,9 @@ def run_ours(args, rank: int, world: int):
     torch.cuda.synchronize()
     ms = t0.elapsed_time(t1) / K
     launches = _lib.PROF.launches
+    # what a caller of the timed path receives from its last step: the computed arrays, not the inputs echoed back
+    # (copied now: the graph's static output buffers are overwritten by the legs below)
+    last = {k: v.detach().clone() for k, v in out.items() if k not in data and torch.is_floating_point(v)} if args.dump_outputs else None
     # ---- leg 2: same K steps with per-kernel CUDA events (roofline of the dominant kernel) ----
     _lib.PROF.reset()
     _lib.PROF.enabled = True
@@ -283,6 +307,8 @@ def run_ours(args, rank: int, world: int):
     }
     if not args.no_cpu_baseline:
         res["cpu_baseline"] = cpu_baseline(cfg, steps=3)
+    if last is not None:
+        dump_outputs(last, args.dump_outputs)
     print(json.dumps(res))
 
 
@@ -637,9 +663,14 @@ def main():
     ap.add_argument("--reps", type=int, default=0, help="N>1: lattice repetitions per box edge instead of the config's own (smaller boxes for tests)")
     ap.add_argument("--no-c4", action="store_true", help="N=8: skip the extra 1M-atom c4 measurement")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from Python instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the outputs of the last one as DIR/<name>.npy "
+                                                             "(float32 / float64; rows of large arrays sampled with a fixed seed, at most "
+                                                             f"{DUMP_BUDGET_BYTES // 10**6} MB of data in all)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs is supported for --impl ours on one GPU")
     if args.impl == "reference":
         return run_reference(args, rank, world)
     if args.impl.startswith("reference-gpu"):

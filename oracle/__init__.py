@@ -15,9 +15,9 @@ PARITY -- what is pinned and what is not:
 * PINNED to the reference's own code: everything mir-group/allegro implements itself
   (allegro/nn/_strided/_contract.py, _channels.py, allegro/nn/_allegro.py, tensorembed.py,
   _edgeembed.py, scalarembed.py, edgewise.py and the assembly in allegro/model/allegro_models.py).
-  ``tests/golden/make_reference_vectors.py`` EXECUTES those unmodified modules from
-  /root/reference in the build container and records inputs, state_dicts and outputs in
-  ``tests/golden/ref_models.pt`` / ``ref_ops.pt``; ``tests/test_reference_golden.py`` checks this
+  ``tests/golden/make_reference_vectors.py`` EXECUTES those unmodified modules from a
+  checkout of the reference and records inputs, state_dicts and outputs in
+  ``tests/golden/ref_models_<k>.pt`` / ``ref_ops_<k>.pt``; ``tests/test_reference_golden.py`` checks this
   oracle against them (strict state_dict load, 1e-12 relative in fp64) on every box.
 * PARITY UNPINNED for the third-party primitives those modules import: e3nn (wigner_3j,
   SphericalHarmonics, Irreps) and nequip (ScalarMLPFunction, Bessel/cutoff embedding,

@@ -1,20 +1,23 @@
-"""Generate golden vectors by EXECUTING THE REFERENCE'S OWN CODE (build container only).
+"""Generate golden vectors by EXECUTING THE REFERENCE'S OWN CODE (needs a checkout of the reference).
 
-    python tests/golden/make_reference_vectors.py        # needs /root/reference
+    python tests/golden/make_reference_vectors.py REFERENCE_CHECKOUT
 
-What runs: the unmodified `allegro/nn/*.py` and `allegro/model/allegro_models.py` from
-/root/reference (mir-group/allegro v0.7.1).  Its third-party imports (e3nn, nequip, hydra) are not
+What runs: the unmodified `allegro/nn/*.py` and `allegro/model/allegro_models.py` from a checkout
+of mir-group/allegro v0.7.1.  Its third-party imports (e3nn, nequip, hydra) are not
 installable in this image, so they resolve to the stand-ins under `tests/golden/_stubs/`, which
 forward to the oracle's restatements of the published algorithms (see `_stubs/README.md` for
 exactly what that does and does not pin).  The reference's package `__init__` (which pulls in the
 nequip-compile tooling) is bypassed by registering a bare parent package; every `allegro.nn` /
 `allegro.model` module is executed as is.
 
-Outputs (committed, small):
-  tests/golden/ref_models.pt   whole-model cases: ctor kwargs, inputs, reference state_dict, outputs
-  tests/golden/ref_ops.pt      operator cases: Contracter / MakeWeightedChannels inputs+outputs,
-                               per-layer irreps of Allegro_Module for a grid of (l_max, parity, L)
+Outputs (committed; each collection is split over numbered files below MAX_FILE_BYTES,
+tests/golden_util.py joins them):
+  tests/golden/ref_models_<k>.pt   whole-model cases: ctor kwargs, inputs, reference state_dict, outputs
+  tests/golden/ref_ops_<k>.pt      operator cases: Contracter / MakeWeightedChannels inputs+outputs,
+                                   per-layer irreps of Allegro_Module for a grid of (l_max, parity, L),
+                                   and a reference model's Contracters as enable_B200Contracter sees them
 """
+import io
 import os
 import sys
 import types
@@ -23,12 +26,13 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+MAX_FILE_BYTES = 900_000
 sys.path.insert(0, os.path.join(HERE, "_stubs"))
 sys.path.insert(0, ROOT)
 
+REF = sys.argv[1] if len(sys.argv) > 1 else ""
 if not os.path.isdir(os.path.join(REF, "allegro")):
-    sys.exit("make_reference_vectors.py needs the reference checkout at /root/reference")
+    sys.exit("usage: make_reference_vectors.py REFERENCE_CHECKOUT (a mir-group/allegro v0.7.1 source tree)")
 _pkg = types.ModuleType("allegro")
 _pkg.__path__ = [os.path.join(REF, "allegro")]
 sys.modules["allegro"] = _pkg
@@ -55,6 +59,31 @@ def pack_state_dict(sd):
         else:
             out[k] = v.clone()
     return out
+
+
+def save_parts(stem, collections):
+    """Write ``collections`` (a dict of lists) as <stem>_1.pt, <stem>_2.pt, ...: records are taken in order and a
+    new file is started before one would exceed MAX_FILE_BYTES.  Returns the file names."""
+    def size(part):
+        buf = io.BytesIO()
+        torch.save(part, buf)
+        return buf.tell()
+
+    parts = [{}]
+    for key, records in collections.items():
+        for rec in records:
+            trial = {k: list(v) for k, v in parts[-1].items()}
+            trial.setdefault(key, []).append(rec)
+            if parts[-1] and size(trial) > MAX_FILE_BYTES:
+                parts.append({key: [rec]})
+            else:
+                parts[-1] = trial
+    names = []
+    for k, part in enumerate(parts, 1):
+        assert size(part) <= MAX_FILE_BYTES, f"one {stem} record alone exceeds {MAX_FILE_BYTES} bytes"
+        names.append(f"{stem}_{k}.pt")
+        torch.save(part, os.path.join(HERE, names[-1]))
+    return names
 
 
 def _cluster(n, box, seed):
@@ -150,7 +179,7 @@ def run_models():
         out.append(rec)
         print(f"{name:28s} atoms {data['pos'].shape[0]:3d} edges {data['edge_index'].shape[1]:5d} E {float(res['total_energy']):+.6f} "
               f"max|F| {float(res['forces'].abs().max()):.4f}")
-    torch.save(out, os.path.join(HERE, "ref_models.pt"))
+    return save_parts("ref_models", {"models": out})
 
 
 def run_ops():
@@ -209,12 +238,24 @@ def run_ops():
                                          int((tp.w3j != 0).sum()), bool(tp.w3j_is_ij_diagonal)) for tp in am.tps],
                                    latent_dims=[tuple(int(w.shape[0]) for w in lat.weights) + (int(lat.weights[-1].shape[1]),) for lat in am.latents]))
     torch.set_default_dtype(prev)
-    torch.save(dict(contracter=contract, channels=channels, layers=layers), os.path.join(HERE, "ref_ops.pt"))
     print(f"operators: {len(contract)} Contracter, {len(channels)} MakeWeightedChannels, {len(layers)} layer-irreps cases")
+    return save_parts("ref_ops", dict(contracter=contract, channels=channels, layers=layers, modifier=[run_modifier()]))
+
+
+def run_modifier():
+    """A model assembled by the reference's builders, as allegro_b200's enable_B200Contracter finds it: the constructor
+    state of every Contracter, the module tree and the state_dict (tests/test_reference_modifier.py)."""
+    kw = dict(seed=3, model_dtype="float64", r_max=4.0, type_names=["H", "C", "O"], l_max=2, num_layers=3, num_scalar_features=16,
+              num_tensor_features=4, avg_num_neighbors=20.0, radial_chemical_embed={"_target_": "allegro.nn.TwoBodyBesselScalarEmbed"})
+    model = allegro.model.AllegroModel(**kw)
+    tps = [dict(irreps_in1=repr(tp.irreps_in1), irreps_in2=repr(tp.irreps_in2), irreps_out=repr(tp.irreps_out), mul=tp.mul,
+                instructions=tp.instructions, path_channel_coupling=tp.path_channel_coupling, scatter_factor=tp.scatter_factor,
+                irrep_normalization=tp.irrep_normalization, num_paths=tp.num_paths, w3j_is_ij_diagonal=bool(tp.w3j_is_ij_diagonal))
+           for tp in model.model.allegro.tps]
+    return dict(kwargs=kw, tps=tps, state_dict=pack_state_dict(model.state_dict()),
+                modules=[(name, type(m).__name__) for name, m in model.named_modules()])
 
 
 if __name__ == "__main__":
-    run_models()
-    run_ops()
-    for f in ("ref_models.pt", "ref_ops.pt"):
+    for f in run_models() + run_ops():
         print(f, os.path.getsize(os.path.join(HERE, f)) // 1024, "KiB")

@@ -1,5 +1,6 @@
 """Loading helpers for the reference-generated fixtures under tests/golden/ (see
 tests/golden/make_reference_vectors.py for how they were produced)."""
+import itertools
 import os
 
 import torch
@@ -20,12 +21,26 @@ def unpack_state_dict(sd):
     return out
 
 
+def _load_parts(stem):
+    """Join <stem>_1.pt, <stem>_2.pt, ... (dicts of lists, split to keep every file small) into one dict of lists."""
+    out = {}
+    for k in itertools.count(1):
+        path = os.path.join(GOLDEN, f"{stem}_{k}.pt")
+        if not os.path.exists(path):
+            break
+        for key, records in torch.load(path, weights_only=False).items():
+            out.setdefault(key, []).extend(records)
+    if not out:
+        raise FileNotFoundError(f"no {stem}_<k>.pt under {GOLDEN}")
+    return out
+
+
 def load_models():
-    return torch.load(os.path.join(GOLDEN, "ref_models.pt"), weights_only=False)
+    return _load_parts("ref_models")["models"]
 
 
 def load_ops():
-    return torch.load(os.path.join(GOLDEN, "ref_ops.pt"), weights_only=False)
+    return _load_parts("ref_ops")
 
 
 def model_case_ids():

@@ -33,3 +33,31 @@ def test_reference_arm_json_line():
 def test_reference_arm_other_ranks_are_silent():
     p = _run({"RANK": "1", "WORLD_SIZE": "2"})
     assert p.returncode == 0 and p.stdout.strip() == ""
+
+
+def test_dump_outputs_dtypes_budget_and_fixed_sample(tmp_path):
+    """bench.py --dump-outputs: float64 stays float64, other floating types become float32, small arrays are written
+    whole, and an array over what is left of the byte budget keeps the same seeded sample of rows on every call."""
+    import numpy as np
+    import torch
+
+    import bench
+
+    g = torch.Generator().manual_seed(1)
+    outs = {"forces": torch.randn(50, 3, generator=g, dtype=torch.float64), "total_energy": torch.randn(1, 1, generator=g, dtype=torch.float64),
+            "edge_features": torch.randn(4000, 16, generator=g).to(torch.bfloat16)}
+    budget = 60_000
+    for d in ("a", "b"):
+        bench.dump_outputs(outs, str(tmp_path / d), budget=budget)
+    got = {p.stem: np.load(p) for p in (tmp_path / "a").iterdir()}
+    assert sorted(got) == sorted(outs)
+    assert got["forces"].dtype == np.float64 and np.array_equal(got["forces"], outs["forces"].numpy())
+    assert got["total_energy"].shape == (1, 1)
+    ef = got["edge_features"]
+    small = outs["forces"].numel() * 8 + 8
+    assert ef.dtype == np.float32 and ef.shape == ((budget - small) // (16 * 4), 16)  # the bytes the small arrays leave
+    assert sum(a.nbytes for a in got.values()) <= budget
+    full = outs["edge_features"].float().numpy()
+    rows = [int(np.flatnonzero((full == r).all(1))[0]) for r in ef]
+    assert rows == sorted(rows) and len(set(rows)) == len(rows)  # distinct rows of the output, in ascending order
+    assert np.array_equal(ef, np.load(tmp_path / "b" / "edge_features.npy"))

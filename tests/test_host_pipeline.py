@@ -4,7 +4,7 @@ The ctypes wrappers of the CUDA kernels (allegro_b200/_lib.py) are replaced by t
 tests/kernel_spec.py (what include/allegro_b200.h says each kernel computes, in torch), and the whole product path --
 AllegroModel state_dict loading, weight folding / packing / column permutations, segment views, the forward and both
 backward orchestrations, CSR and edge permutations, scale/shift, stress -- is compared with vectors produced by the
-reference's own code (tests/golden/ref_models.pt).  A mismatch here is a bug in the Python side of the product (or in the
+reference's own code (tests/golden/ref_models_<k>.pt).  A mismatch here is a bug in the Python side of the product (or in the
 kernel contract), independent of any CUDA kernel; the kernels themselves are checked on the GPU.
 """
 import pytest

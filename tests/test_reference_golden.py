@@ -1,10 +1,10 @@
 """Oracle and product host logic against vectors produced by the REFERENCE'S OWN CODE.
 
-tests/golden/ref_models.pt / ref_ops.pt were written by tests/golden/make_reference_vectors.py, which
-executes the unmodified /root/reference allegro/nn + allegro/model modules (third-party e3nn / nequip
+tests/golden/ref_models_<k>.pt / ref_ops_<k>.pt were written by tests/golden/make_reference_vectors.py, which
+executes the reference's unmodified allegro/nn + allegro/model modules (third-party e3nn / nequip
 calls resolved to stand-ins backed by the oracle's primitives, tests/golden/_stubs/README.md).  These
 tests therefore pin the oracle's restatement -- and the product's table / irreps / state_dict logic --
-to the reference implementation itself, on every box (no /root/reference needed at test time).
+to the reference implementation itself, on every machine (no reference checkout needed at test time).
 
 fp64 cases must agree to rounding (1e-12 relative), the fp32 case to 1e-5.
 """
